@@ -4,7 +4,7 @@
 Metric (BASELINE.json): Mcells/s of slope + hillshade + focal.mean on a float32 DEM, with the
 fraction of the HBM roofline, at 1/2/4/8 GPUs.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--raster R]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--raster R] [--dump-outputs DIR]
 
 N = 1   : 32768 x 32768 synthetic fBm-like DEM resident on the GPU (BASELINE configs[1]).
 N > 1   : launched by torchrun, one rank per GPU; a 65536 x 65536 DEM (configs[4]) is row-striped
@@ -33,6 +33,11 @@ and
                   a same-raster anchor.
 
 --impl reference times that CPU oracle instead (all host threads, bounded sample per step).
+
+--dump-outputs DIR (N = 1) writes the slope, hillshade and mean rasters of the last timed step as
+DIR/<name>.npy (float32), on a fixed, seeded grid of at most 2048 interior rows x 2048 interior
+columns (48 MiB in all).  The edge rows and columns are NaN by design and are not written.  The DEM is
+a pure function of its seed, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -232,6 +237,32 @@ def event_times(fn, steps, warmup=3):
     return float(np.median(t)), t
 
 
+DUMP_SIDE = 2048   # sampled rows x columns per array: 3 float32 arrays of 2048^2 are 48 MiB
+
+
+def dump_sample(n, side=DUMP_SIDE, seed=0):
+    """Sorted indices of a fixed, seeded sample of at most `side` of the interior indices 1 .. n - 2.
+    The first and last row and column are left out: the 3x3 operators make them NaN by design (the
+    reference's raster-edge rule, which the test suite checks), and the dump holds finite values only."""
+    inner = np.arange(1, n - 1)
+    if len(inner) <= side:
+        return inner
+    return np.sort(np.random.default_rng(seed).choice(inner, side, replace=False))
+
+
+def dump_outputs(out_dir, outs):
+    """--dump-outputs: the arrays of the last timed step, as out_dir/<name>.npy, sampled on a fixed grid
+    of interior rows x columns, the same for every run and build."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outs.items():
+        rows = torch.from_numpy(dump_sample(t.shape[0])).to(t.device)
+        cols = torch.from_numpy(dump_sample(t.shape[1])).to(t.device)
+        a = t[rows[:, None], cols[None, :]].cpu().numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def rel_err(got, ref, rtol=1e-5, atol=1e-6, circular=False):
     """worst |got - ref| / (rtol |ref| + atol) with identical NaN masks (raises otherwise)."""
     g = np.asarray(got, dtype=np.float64)
@@ -324,6 +355,8 @@ def run_gpu_arm(args):
     t_end.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs)
     total_ms = t_begin.elapsed_time(t_end)
     kt = np.array([[e[j].elapsed_time(e[j + 1]) for j in range(3)] for e in ev])  # ms per kernel
     if world > 1:
@@ -809,7 +842,15 @@ def main():
                     help="profiling runs only: skip the per-operator record and the 65536^2 anchor")
     ap.add_argument("--skip-host", action="store_true",
                     help="profiling runs only: skip the e2e (host-buffer) and CPU-baseline legs")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy, sampled on a fixed, seeded "
+                         "grid of at most %d interior rows x columns (the NaN edge rows and columns are left out)"
+                         % DUMP_SIDE)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1 or int(os.environ.get("WORLD_SIZE", "1")) != 1):
+        ap.error("--dump-outputs is supported on the single-GPU run only")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

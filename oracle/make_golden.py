@@ -1,6 +1,6 @@
 """Generate tests/golden/*.npz from the UNMODIFIED reference (run in the build container only).
 
-TEST INFRASTRUCTURE.  Two fixture files are produced:
+TEST INFRASTRUCTURE.  Three fixture files are produced:
 
 * tests/golden/known_answers.npz -- the literal known-answer arrays that the reference's
   own test-suite holds for the hot path (QGIS / hand-derived tables; SURVEY.md 8c).  They are
@@ -9,6 +9,8 @@ TEST INFRASTRUCTURE.  Two fixture files are produced:
 * tests/golden/reference_outputs.npz -- seeded inputs and the outputs of the reference's
   Numba-CPU / NumPy kernels (loaded through oracle/ref_loader.py) on those inputs, for every
   op on the hot path, including NaN-laden, flat ("water"), integer-valued and odd-shaped cases.
+* tests/golden/reference_signatures.json -- parameter names, order and defaults of every public
+  function on the path, read with `inspect` from the reference modules.
 
 Usage:  python oracle/make_golden.py         (needs /root/reference)
 """
@@ -344,13 +346,50 @@ def reference_outputs():
     return g
 
 
+# ------------------------------------------------------------------ public signatures
+SIGNATURES = {'slope': ['slope'], 'aspect': ['aspect'], 'curvature': ['curvature'], 'hillshade': ['hillshade'],
+              'focal': ['mean', 'apply', 'focal_stats', 'hotspots'],
+              'convolution': ['convolve_2d', 'convolution_2d', 'custom_kernel', 'circle_kernel', 'annulus_kernel',
+                              'calc_cellsize'],
+              'zonal': ['stats', 'crosstab'], 'analytics': ['summarize_terrain'],
+              'multispectral': ['ndvi', 'savi', 'evi', 'arvi', 'gci', 'sipi', 'ebbi', 'nbr', 'nbr2', 'ndmi'],
+              'utils': ['get_dataarray_resolution', 'calc_res', 'validate_arrays']}
+
+
+def _param(name, default):
+    """One parameter as JSON: no "default" key when it has none; a callable default by its
+    __name__, a NaN default as a flag, any other default by its repr."""
+    import inspect
+    if default is inspect.Parameter.empty:
+        return {"name": name}
+    if callable(default):
+        return {"name": name, "callable": getattr(default, "__name__", None)}
+    if isinstance(default, float) and default != default:
+        return {"name": name, "nan": True}
+    return {"name": name, "repr": repr(default)}
+
+
+def reference_signatures():
+    import inspect
+    sigs = {}
+    for mod, names in SIGNATURES.items():
+        m = ref_loader.load(mod)
+        sigs[mod] = {n: [_param(k, v.default) for k, v in inspect.signature(inspect.unwrap(getattr(m, n))).parameters.items()]
+                     for n in names}
+    return sigs
+
+
 def main():
+    import json
     os.makedirs(OUT_DIR, exist_ok=True)
     ka = known_answers()
     np.savez_compressed(os.path.join(OUT_DIR, "known_answers.npz"), **ka)
     ro = reference_outputs()
     np.savez_compressed(os.path.join(OUT_DIR, "reference_outputs.npz"), **ro)
-    for n in ("known_answers.npz", "reference_outputs.npz"):
+    with open(os.path.join(OUT_DIR, "reference_signatures.json"), "w") as f:
+        json.dump(reference_signatures(), f, indent=1)
+        f.write("\n")
+    for n in ("known_answers.npz", "reference_outputs.npz", "reference_signatures.json"):
         print(n, os.path.getsize(os.path.join(OUT_DIR, n)), "bytes")
     print(len(ka), "known-answer arrays;", len(ro), "reference input/output arrays")
 

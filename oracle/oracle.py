@@ -11,29 +11,44 @@ multispectral._*_cpu, zonal._stats_numpy.
 import ctypes
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _SO = os.path.join(_HERE, "libxrs_oracle.so")
 _lib = None
+_tmp_so = None      # build()'s product when the tree is read-only
 
 STAT_IDS = {"mean": 0, "sum": 1, "min": 2, "max": 3, "std": 4, "range": 5, "var": 6}
 
 
 def build(force=False):
+    """Returns the path of an up-to-date libxrs_oracle.so: the in-tree one, rebuilt if it is older than
+    its source; in a temporary directory instead when the tree is read-only (bench.py must run there)."""
+    global _tmp_so
     src = os.path.join(_HERE, "xrs_oracle.c")
-    if force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src):
-        subprocess.check_call(["make", "-C", _HERE, "-B", "libxrs_oracle.so"],
-                              stdout=subprocess.DEVNULL)
-    return _SO
+    stale = force or not os.path.exists(_SO) or os.path.getmtime(_SO) < os.path.getmtime(src)
+    if not stale:
+        return _SO
+    if os.access(_HERE, os.W_OK):
+        out_dir = _HERE
+    elif _tmp_so is not None and not force:
+        return _tmp_so
+    else:
+        out_dir = tempfile.mkdtemp(prefix="xrs_oracle_")
+    subprocess.check_call(["make", "-f", os.path.join(_HERE, "Makefile"), "-C", out_dir, "-B", "VPATH=" + _HERE,
+                           "libxrs_oracle.so"], stdout=subprocess.DEVNULL)
+    so = os.path.join(out_dir, "libxrs_oracle.so")
+    if out_dir != _HERE:
+        _tmp_so = so
+    return so
 
 
 def lib():
     global _lib
     if _lib is None:
-        build()
-        _lib = ctypes.CDLL(_SO)
+        _lib = ctypes.CDLL(build())
     return _lib
 
 

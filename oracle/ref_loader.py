@@ -2,9 +2,8 @@
 
 TEST INFRASTRUCTURE -- never imported by the product path, by bench.py's GPU arm
 or by anything that runs on the GPU box (where /root/reference does not exist).
-It is used (a) by oracle/make_golden.py to generate tests/golden/*.npz and
-(b) by tests marked ``needs_reference`` to pin the C oracle against the real
-reference when the reference tree is present.
+It is used only by oracle/make_golden.py to generate the fixtures under tests/golden/;
+the tests read those fixtures and never the reference itself.
 
 `import xrspatial` fails here because xarray / datashader are not installed
 (xrspatial/utils.py:6-9), so we register stub modules for those two packages and a

@@ -1,3 +1,4 @@
+import json
 import os
 import sys
 
@@ -14,15 +15,6 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box)")
-    config.addinivalue_line("markers", "needs_reference: needs /root/reference (build container only)")
-
-
-def pytest_collection_modifyitems(config, items):
-    have_ref = os.path.isdir("/root/reference/xrspatial")
-    skip_ref = pytest.mark.skip(reason="/root/reference not present")
-    for item in items:
-        if "needs_reference" in item.keywords and not have_ref:
-            item.add_marker(skip_ref)
 
 
 @pytest.fixture(scope="session")
@@ -33,3 +25,9 @@ def known():
 @pytest.fixture(scope="session")
 def refout():
     return dict(np.load(os.path.join(GOLDEN, "reference_outputs.npz"), allow_pickle=False))
+
+
+@pytest.fixture(scope="session")
+def refsig():
+    with open(os.path.join(GOLDEN, "reference_signatures.json")) as f:
+        return json.load(f)

@@ -3,8 +3,9 @@ the product refuses to run without a CUDA device (no CPU fallback)."""
 import ctypes
 import os
 import re
+import subprocess
+import sys
 
-import numpy as np
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -41,15 +42,23 @@ def test_ctypes_prototypes_cover_the_header():
 
 
 def test_no_cpu_fallback_without_gpu():
-    torch = pytest.importorskip("torch")
-    if torch.cuda.is_available():
-        pytest.skip("a GPU is present")
-    import xrspatial_b200 as xb
-    agg = xb.DataArray(np.zeros((8, 8), np.float32), attrs={"res": (1, 1)})
-    with pytest.raises(RuntimeError):
-        xb.slope(agg)          # host path needs the device: fails loudly
-    with pytest.raises(RuntimeError):
-        xb.ndvi(agg, agg)
+    """The host path needs the device and fails loudly without one.  Checked in a fresh interpreter that
+    sees no CUDA device, so that GPU hosts check it too."""
+    pytest.importorskip("torch")
+    code = "\n".join([
+        "import numpy as np",
+        "import xrspatial_b200 as xb",
+        "agg = xb.DataArray(np.zeros((8, 8), np.float32), attrs={'res': (1, 1)})",
+        "for name, f in (('slope', lambda: xb.slope(agg)), ('ndvi', lambda: xb.ndvi(agg, agg))):",
+        "    try:",
+        "        f()",
+        "    except RuntimeError:",
+        "        continue",
+        "    raise SystemExit('%s computed without a CUDA device' % name)",
+    ])
+    env = dict(os.environ, CUDA_VISIBLE_DEVICES="")
+    r = subprocess.run([sys.executable, "-s", "-c", code], cwd=ROOT, env=env, capture_output=True, text=True)
+    assert r.returncode == 0, r.stdout + r.stderr
 
 
 def test_argument_errors_do_not_need_a_gpu():

@@ -195,41 +195,37 @@ def test_crosstab_pivot_matches_pair_loop():
         np.testing.assert_array_equal(counts, c2)
 
 
-@pytest.mark.needs_reference
-def test_public_signatures_equal_the_reference():
-    """Parameter names, order and defaults of every public function on the path, read with `inspect`
-    from the unmodified reference (loaded through oracle/ref_loader.py) and from this package.  The only
-    allowed difference: a trailing `comm=None` (row-stripe group) on the zonal functions."""
+def test_public_signatures_equal_the_reference(refsig):
+    """Parameter names, order and defaults of every public function on the path: the reference's, read with
+    `inspect` from the unmodified reference by oracle/make_golden.py (tests/golden/reference_signatures.json),
+    and this package's.  The only allowed difference: a trailing `comm=None` (row-stripe group) on the zonal
+    functions."""
     import importlib
     import inspect
-    import ref_loader
-    table = {'slope': ['slope'], 'aspect': ['aspect'], 'curvature': ['curvature'], 'hillshade': ['hillshade'],
-             'focal': ['mean', 'apply', 'focal_stats', 'hotspots'],
-             'convolution': ['convolve_2d', 'convolution_2d', 'custom_kernel', 'circle_kernel', 'annulus_kernel',
-                             'calc_cellsize'],
-             'zonal': ['stats', 'crosstab'], 'analytics': ['summarize_terrain'],
-             'multispectral': ['ndvi', 'savi', 'evi', 'arvi', 'gci', 'sipi', 'ebbi', 'nbr', 'nbr2', 'ndmi'],
-             'utils': ['get_dataarray_resolution', 'calc_res', 'validate_arrays']}
+    assert sum(len(v) for v in refsig.values()) == 30
 
     def params(f):
         return [(k, v.default) for k, v in inspect.signature(inspect.unwrap(f)).parameters.items()]
 
-    for mod, names in table.items():
-        ref_mod = ref_loader.load(mod)
+    for mod, funcs in refsig.items():
         mine_mod = importlib.import_module('xrspatial_b200.' + mod)
-        for n in names:
-            rp, mp = params(getattr(ref_mod, n)), params(getattr(mine_mod, n))
+        for n, rp in funcs.items():
+            mp = params(getattr(mine_mod, n))
             if mod == 'zonal':
                 assert mp[-1] == ('comm', None), n
                 mp = mp[:-1]
-            assert [k for k, _ in rp] == [k for k, _ in mp], (mod, n)
-            for (k, a), (_, b) in zip(rp, mp):
-                if callable(a) or callable(b):
-                    assert getattr(a, '__name__', a) == getattr(b, '__name__', b) or callable(a) == callable(b), (mod, n, k)
-                elif isinstance(a, float) and a != a:
-                    assert b != b
+            assert [r['name'] for r in rp] == [k for k, _ in mp], (mod, n)
+            for r, (k, b) in zip(rp, mp):
+                if set(r) == {'name'}:                      # no default
+                    assert b is inspect.Parameter.empty, (mod, n, k)
+                elif 'callable' in r:
+                    assert callable(b) or r['callable'] == getattr(b, '__name__', b), (mod, n, k)
+                elif callable(b):
+                    assert r.get('repr') == repr(b.__name__), (mod, n, k)
+                elif r.get('nan'):
+                    assert b != b, (mod, n, k)
                 else:
-                    assert repr(a) == repr(b), (mod, n, k, a, b)
+                    assert r['repr'] == repr(b), (mod, n, k, r['repr'], b)
 
 
 # ----------------------------------------------------------------- the xarray facade (_xr.py)
